@@ -63,7 +63,26 @@ def parse_args():
     ap.add_argument("--groups", type=int, default=0, help="force the window-group count of the pipeline (0 = automatic)")
     ap.add_argument("--configs", action="store_true",
                     help="instead of the headline line: time every BASELINE.json config on one GPU (one JSON line, key `configs`)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the result of the last timed step as DIR/<name>.npy (float64), to compare two builds output for "
+                         "output; the inputs depend only on the arguments")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.configs):
+        ap.error("--dump-outputs applies to the headline GPU run (not --impl reference or --configs)")
+    return args
+
+
+def dump_outputs(dirname, xy: bytes, is_inf: int):
+    """What nmsm_msm_device hands its caller for one BLS12-381 G1 MSM: the affine result (x, y), each 48 bytes little-endian,
+    stored as 12 little-endian 32-bit limbs per coordinate (exact in float64), and the point-at-infinity flag."""
+    import numpy as np
+
+    os.makedirs(dirname, exist_ok=True)
+    limbs = np.frombuffer(xy, dtype="<u4").reshape(2, POINT_BYTES // 8)
+    np.save(os.path.join(dirname, "msm_affine_xy_limbs.npy"), limbs.astype(np.float64))
+    np.save(os.path.join(dirname, "msm_is_infinity.npy"), np.array([is_inf], dtype=np.float64))
 
 
 # --------------------------------------------------------------------------------------------
@@ -432,6 +451,7 @@ def main():
     barrier()
     elapsed = max_over_ranks(time.perf_counter() - t0)
     check_result()
+    last_xy, last_inf = out.raw, inf.value  # `out` is reused by the companion measurements below
     main_info = nmsm.last_timing()[1]
     device_ms = max_over_ranks(sum(dev_ms) / len(dev_ms))
     value = n_total * args.steps / elapsed
@@ -669,6 +689,8 @@ def main():
         "fixed_base": fixed,
         "any_point": any_point,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_xy, last_inf)
     _emit(real_stdout, line)
     if world > 1:
         dist.destroy_process_group()
